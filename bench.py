@@ -40,7 +40,7 @@ CONFIGS = {
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=3, help="timed passes over the request set")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--model", default="preset:qwen3-8b")
@@ -64,6 +64,9 @@ def parse():
     ap.add_argument("--fixed-prompts", action="store_true",
                     help="re-use the same token ids in every pass (with prefix caching the prompts of later passes "
                          "would then be served from the cache: NOT the benchmark; for debugging only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed passes, write what the last pass returned (generated token ids) as "
+                         "DIR/*.npy, so that two builds can be compared output for output")
     return ap.parse_args()
 
 
@@ -157,6 +160,28 @@ def synth_requests(n, vocab, seed, pass_idx=0):
     trng = np.random.default_rng([seed, 7919, pass_idx])
     prompts = [trng.integers(10, vocab - 10, size=p).tolist() for p in lens]
     return prompts, outs
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, seqs, seed):
+    """Write what `LLM.generate` returned to its caller in one pass: the generated token ids of every request,
+    concatenated in request order (`output_token_ids.npy`), how many each request generated (`output_lens.npy`) and
+    which requests these are (`request_index.npy`). float64 holds token ids exactly. When the whole set would exceed
+    64 MB, a fixed sample of requests drawn with `seed` is written instead."""
+    import numpy as np
+    gen = [np.asarray(q.token_ids[q.prompt_len:], dtype=np.float64) for q in seqs]
+    idx = np.arange(len(gen))
+    if sum(g.nbytes + 16 for g in gen) > DUMP_LIMIT_BYTES:
+        order = np.random.default_rng([seed, 4099]).permutation(len(gen))
+        sizes = np.cumsum([gen[i].nbytes + 16 for i in order])
+        idx = np.sort(order[:int(np.searchsorted(sizes, DUMP_LIMIT_BYTES, side="right"))])
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "output_token_ids.npy"),
+            np.concatenate([gen[i] for i in idx]) if len(idx) else np.zeros(0, np.float64))
+    np.save(os.path.join(out_dir, "output_lens.npy"), np.array([len(gen[i]) for i in idx], dtype=np.float64))
+    np.save(os.path.join(out_dir, "request_index.npy"), idx.astype(np.float64))
 
 
 class ClockSampler(threading.Thread):
@@ -256,7 +281,7 @@ def main():
     runner = llm.worker.runner
 
     # token ids of every pass prepared up front (host work outside the timed region; the reference arm does the same)
-    n_pass = args.warmup + 2 * args.steps
+    n_pass = args.warmup + args.steps
     pass_prompts = [prompts if (args.fixed_prompts or i == 0) else synth_requests(args.num_prompts, vocab, args.seed, i)[0]
                     for i in range(n_pass)]
     if cpu_selftest:
@@ -277,10 +302,9 @@ def main():
     for _ in range(args.warmup):
         one_pass()
 
-    # ---- region A: K passes through the public API (LLM.generate: every iteration copies its batch arrays
-    # host->device from pinned memory and reads the sampled tokens back), bracketed by barrier + sync and timed with
-    # CUDA events on the launching stream -> `value`. Region B below repeats K passes under the host's wall clock
-    # -> `e2e` (an independent measurement, not the same bracket read with a second clock).
+    # ---- the K timed passes through the public API (LLM.generate: every iteration copies its batch arrays
+    # host->device from pinned memory and reads the sampled tokens back), bracketed by barrier + sync. CUDA events on
+    # the launching stream -> `value`; the host's wall clock around the same bracket -> `e2e`.
     sampler = ClockSampler(int(os.environ.get("LOCAL_RANK", "0"))) if rank == 0 else None
     if sampler:
         sampler.start()
@@ -289,9 +313,8 @@ def main():
     stats0 = dict(runner.stats)
     launches0 = sm100.launches()
     barrier()
-    if cpu_selftest:
-        th0 = time.perf_counter()
-    else:
+    t0 = time.perf_counter()
+    if not cpu_selftest:
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         ev0.record()
     seqs = None
@@ -300,18 +323,12 @@ def main():
     if not cpu_selftest:
         ev1.record()
     barrier()
-    dev_ms = (time.perf_counter() - th0) * 1e3 if cpu_selftest else ev0.elapsed_time(ev1)
+    wall_s = time.perf_counter() - t0
+    dev_ms = wall_s * 1e3 if cpu_selftest else ev0.elapsed_time(ev1)
     busy_ms = runner.gpu_busy_ms()
     runner.time_steps = False
     stats1 = dict(runner.stats)
     launches = (sm100.launches() - launches0) + (stats1["graph_kernel_launches"] - stats0["graph_kernel_launches"])
-    # ---- region B: end to end through the public API, wall clock ----
-    barrier()
-    t0 = time.perf_counter()
-    for _ in range(args.steps):
-        seqs = one_pass()
-    barrier()
-    wall_s = time.perf_counter() - t0
     if sampler:
         sampler.stop()
     if world > 1:
@@ -319,6 +336,8 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         dev_ms, wall_ms, busy_ms = t.tolist()
         wall_s = wall_ms / 1e3
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, seqs, args.seed)
     if rank == 0:
         value = args.steps * total_out / (dev_ms / 1e3)
         e2e = args.steps * total_out / wall_s
@@ -329,7 +348,7 @@ def main():
         except Exception:  # noqa: BLE001
             pass
         eng_steps = stats1["steps"] - stats0["steps"]
-        # request latencies of the last end-to-end pass (all requests arrive together at t0: offline workload)
+        # request latencies of the last timed pass (all requests arrive together at t0: offline workload)
         lat = None
         try:
             ttft = sorted((q.first_token_time - q.arrival_time) * 1e3 for q in seqs if q.first_token_time)
@@ -337,7 +356,7 @@ def main():
                           for q in seqs if q.first_token_time and q.finish_time and q.num_output_tokens > 1)
             lat = {"p50_ttft_ms": round(ttft[len(ttft) // 2], 1), "p99_ttft_ms": round(ttft[int(len(ttft) * 0.99)], 1),
                    "p50_tpot_ms": round(tpot[len(tpot) // 2], 2), "p99_tpot_ms": round(tpot[int(len(tpot) * 0.99)], 2),
-                   "arrival": "all requests at t0 (offline batch)", "source": "last end-to-end pass"}
+                   "arrival": "all requests at t0 (offline batch)", "source": "last timed pass"}
         except Exception:  # noqa: BLE001
             pass
         out = {

@@ -400,8 +400,12 @@ class CausalLM(nn.Module):
 
     def init_dummy(self, seed: int = 0):
         """`--load-format dummy`: random weights of the right shapes (reference: model_loader.py:154)."""
-        g = torch.Generator(device="cpu").manual_seed(seed + 1000 * self.tp_rank + 7 * ps.get_pp_rank())
+        rank_seed = seed + 1000 * self.tp_rank + 7 * ps.get_pp_rank()
+        g = torch.Generator(device="cpu").manual_seed(rank_seed)
+        gd = None    # seeded on-device RNG: the same dummy weights in every run, so that runs can be compared
         for name, p in self.named_parameters():
+            if p.is_cuda and gd is None:
+                gd = torch.Generator(device=p.device).manual_seed(rank_seed)
             if name.endswith("norm_w"):
                 p.data.fill_(1.0)
             elif p.dim() == 1:
@@ -415,12 +419,13 @@ class CausalLM(nn.Module):
                 flat = p.data.view(-1)
                 for s0 in range(0, flat.numel(), step):
                     e0 = min(s0 + step, flat.numel())
-                    flat[s0:e0].copy_((torch.randn(e0 - s0, device=p.device) * 100.0).clamp_(-448.0, 448.0)
+                    flat[s0:e0].copy_((torch.randn(e0 - s0, device=p.device, generator=gd if p.is_cuda else None)
+                                       * 100.0).clamp_(-448.0, 448.0)
                                      .to(torch.float8_e4m3fn))   # e4m3fn has no inf: out-of-range casts give NaN
             elif name.endswith("_ws"):
                 p.data.fill_(0.02 / 100.0)
             elif p.is_cuda:
-                p.data.normal_(mean=0.0, std=0.02)  # on-device RNG: 8B params in well under a second
+                p.data.normal_(mean=0.0, std=0.02, generator=gd)  # on-device RNG: 8B params in well under a second
             else:
                 flat = p.data.view(-1)
                 step = 1 << 24

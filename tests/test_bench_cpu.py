@@ -39,6 +39,22 @@ def test_bench_contract_single_process():
     assert kinds == {} or all(len(v) == 3 for v in kinds.values())
 
 
+def test_bench_dump_outputs_are_reproducible(tmp_path):
+    """`--dump-outputs DIR`: the generated token ids of the last timed pass, as float .npy files, identical when the
+    same arguments run again."""
+    import numpy as np
+    runs = []
+    for name in ("a", "b"):
+        d = _run(["--dump-outputs", str(tmp_path / name)])
+        runs.append({k: np.load(tmp_path / name / f"{k}.npy")
+                     for k in ("output_token_ids", "output_lens", "request_index")})
+    a, b = runs
+    for k in a:
+        assert a[k].dtype == np.float64 and np.array_equal(a[k], b[k]), k
+    assert a["request_index"].tolist() == list(range(6)) and a["output_lens"].sum() == a["output_token_ids"].size
+    assert a["output_token_ids"].size == d["config"]["output_tokens_per_step"]
+
+
 def test_bench_contract_two_ranks_and_named_config():
     d = _run(["--config", "mixtral-8x7b-ep"], nproc=2)
     assert d["n_gpus"] == 2 and d["config"]["parallelism"] == "tp2" and d["value"] > 0
